@@ -1,13 +1,13 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200 build (contract: see the task statement / DESIGN.md §4).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (N=1): BASELINE.json configs[1] — FP8 paged decode attention, q per-token/head scales,
 k/v per-tensor scales, bs=64, GQA 32/8, d=128, seq=8192, page 64, synthetic data.
 A step = one decode-attention pass over that batch: task-map assign + split-k attention + combine.
 
-  value      tokens/s with every input already resident in HBM (CUDA events, K steps).
+  value      tokens/s with every input already resident in HBM (CUDA events, one region of K steps).
   e2e        the same through the public API with HOST inputs: per step the pinned host q, q scales,
              kv lengths and page table are copied H2D, the task map is assigned, attention runs, and
              the bf16 output is read back D2H (the paged KV cache is device-resident state, exactly
@@ -25,6 +25,9 @@ sharded path, fuse_allreduce_rmsnorm, runs at W=N inside `extra.allreduce_c5` (h
 low-latency kernels over the NCCL-initialised symmetric buffers, CUDA-graph timed, max over ranks).
 `--impl reference`: times the reference's own algorithm on the host cores (the torch CPU reference
 path restated in oracle/, since the reference's sm_90a build cannot execute on sm_100).
+`--dump-outputs DIR`: after the timed steps, rank 0 writes the bf16 attention output of the last
+step as DIR/attention_decode_fp8_output.npy (float32, [64, 32, 128]). The inputs are seeded, so
+two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -198,6 +201,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=None)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-extra", action="store_true", help="skip the `extra` block (C3/C4/C5/route GEMM)")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, default=None,
+                    help="write the attention output of the last timed step to DIR as .npy")
     a = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -205,6 +210,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
 
     if a.impl == "reference":
+        if a.dump_outputs is not None:
+            ap.error("--dump-outputs applies to --impl b200")
         a.steps = a.steps or 3
         a.warmup = 1 if a.warmup is None else a.warmup
         run_reference(a, rank, world)
@@ -253,27 +260,27 @@ def main():
         sampler.start()
 
     # ---------------- value: inputs resident in HBM ----------------
-    # Each timed region is EXACTLY K steps between barrier + synchronize; short runs (small K) are
-    # repeated until >= 200 steps have been timed and the median region is reported.
+    # One timed region of exactly K steps between barrier + synchronize.
     for _ in range(a.warmup):
         step_resident()
-    repeats = max(1, -(-200 // a.steps))
-    region_ms = []
-    for _ in range(repeats):
-        barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(a.steps):
-            step_resident()
-        e1.record()
-        barrier()
-        t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
-        if dist is not None:
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        region_ms.append(float(t.item()))
-    ms_total = sorted(region_ms)[len(region_ms) // 2]
+    barrier()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(a.steps):
+        step_resident()
+    e1.record()
+    barrier()
+    t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
+    if dist is not None:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    ms_total = float(t.item())
     ms_per_step = ms_total / a.steps
     value = world * B * Sq / (ms_per_step * 1e-3)
+    if a.dump_outputs is not None and rank == 0:
+        import numpy as np
+
+        a.dump_outputs.mkdir(parents=True, exist_ok=True)
+        np.save(a.dump_outputs / "attention_decode_fp8_output.npy", out.float().cpu().numpy())
 
     # ---------------- roofline: the attention kernel alone ----------------
     y, args, keep = hatt._decode_fp8_prepare(
@@ -375,8 +382,6 @@ def main():
             "warmup": a.warmup, "ms_per_step": ms_per_step, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "fp8_e4m3 (fp32 accumulate)",
             "data": "synthetic", "config": config_dict(world),
-            "timed_regions": {"count": repeats, "steps_each": a.steps,
-                              "ms_min": min(region_ms), "ms_median": ms_total, "ms_max": max(region_ms)},
             "roofline": {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s",
                          "frac": achieved / peak, "traffic": traffic,
                          "traffic_source": "profiles/decode_attn_traffic.json (one ncu --set full capture)",
@@ -454,8 +459,10 @@ def main():
             dist.destroy_process_group()
         except Exception:  # noqa: BLE001
             pass
-    sys.stdout.flush()
-    os._exit(0)  # symmetric-memory handles and NCCL teardown order must not turn a finished run into a hang
+        sys.stdout.flush()
+        # with several ranks, symmetric-memory handles and NCCL teardown order must not turn a
+        # finished run into a hang; a single process returns normally
+        os._exit(0)
 
 
 if __name__ == "__main__":

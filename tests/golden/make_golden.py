@@ -1,7 +1,7 @@
 """Generate the golden fixtures in tests/golden/ from the REFERENCE's own code.
 
-Run in the build container only (needs /root/reference; the GPU box never runs this):
-    python tests/golden/make_golden.py
+Needs a checkout of the original hpc-ops sources; the tests only read the stored fixtures:
+    python tests/golden/make_golden.py <hpc-ops checkout>
 
 * attention: the reference keeps its ground truth as pure-torch functions inside its test files.
   Those files `import hpc` at module level (needs their CUDA build), so we AST-extract the
@@ -11,7 +11,10 @@ Run in the build container only (needs /root/reference; the GPU box never runs t
   reference (assign_task.cu:424 `TaskScheduleInfo task_info;`) and are stored zeroed.
 """
 import ast
+import json
 import math
+import re
+import subprocess
 import sys
 from pathlib import Path
 
@@ -19,7 +22,7 @@ import numpy as np
 import torch
 
 REPO = Path(__file__).resolve().parents[2]
-REF = Path("/root/reference")
+REF = None  # the original project's checkout, from the command line
 OUT = Path(__file__).resolve().parent
 sys.path.insert(0, str(REPO))
 
@@ -169,6 +172,42 @@ def taskmap_cases():
     print("wrote taskmap_ref", len(cases))
 
 
+def taskmap_random_cases():
+    """Random configurations with the new token included. Their task maps come to ~15M rows, so
+    each is stored as its row count and `taskmap_digest`; `lens` holds the cases' lengths back to
+    back, `cfg` rows are [B, H, sq, tilen, ctas, mpl]."""
+    assert otm.ref_lib() is not None, "oracle/_ref not built"
+    sys.path.insert(0, str(OUT.parent))
+    from test_oracle_taskmap import _random_cases, taskmap_digest
+    lens, cfg, rows, sha = [], [], [], []
+    for ln, ctas, H, sq, tilen, inc, mpl in _random_cases(300, 2):
+        if inc:
+            ref = otm.assign_ref(ln, ctas, H, sq, tilen, inc, mpl)
+            lens.append(np.asarray(ln, np.int32))
+            cfg.append([len(ln), H, sq, tilen, ctas, mpl])
+            rows.append(ref.shape[0])
+            sha.append(taskmap_digest(ref))
+    np.savez_compressed(OUT / "taskmap_ref_random.npz", lens=np.concatenate(lens),
+                        cfg=np.array(cfg, np.int32), rows=np.array(rows), sha256=np.stack(sha))
+    print("wrote taskmap_ref_random", len(cfg))
+
+
+def schemas():
+    """Schema of every in-scope op, parsed out of the reference's `m.def("name(...) -> ...")`."""
+    sys.path.insert(0, str(OUT.parent))
+    from test_api_surface import IN_SCOPE_OPS
+    out = {}
+    for f in sorted(REF.glob("src/**/*.cc")):
+        text = f.read_text(errors="ignore")
+        for m in re.finditer(r"m\.def\(\s*((?:\"(?:[^\"\\]|\\.)*\"\s*)+)[,)]", text):
+            schema = "".join(re.findall(r"\"((?:[^\"\\]|\\.)*)\"", m.group(1)))
+            if "(" in schema:
+                out[schema.split("(", 1)[0].strip()] = schema
+    keep = {n: out[n] for n in IN_SCOPE_OPS if n in out}
+    (OUT / "reference_schemas.json").write_text(json.dumps(keep, indent=1) + "\n")
+    print("wrote reference_schemas", len(keep))
+
+
 class _TorchCPU:
     """`torch` stand-in for exec'ing reference test functions that hard-code device="cuda"."""
 
@@ -315,6 +354,8 @@ def group_gemm_cases():
 
 
 if __name__ == "__main__":
+    REF = Path(sys.argv[1]).resolve()
+    subprocess.run(["make", "-C", str(REPO / "oracle"), "ref", f"REF={REF}"], check=True)
     allreduce_case("w4", 4, 13, 512, 10001)
     group_gemm_cases()
     act_case("a", 64, 256, 41)
@@ -333,3 +374,5 @@ if __name__ == "__main__":
     decode_bf16_case("b3_bs16_nhd", 3, 2, [70, 129, 300], 1, 8, 16, 41, "NHD")
     decode_bf16_case("b4_bs64_hnd", 4, 1, [1, 64, 65, 260], 2, 8, 64, 10086, "HND")
     taskmap_cases()
+    taskmap_random_cases()
+    schemas()
