@@ -266,6 +266,10 @@ __device__ __forceinline__ void tma_prefetch_l2_3d(const CUtensorMap* map, int c
                "r"(c0), "r"(c1), "r"(c2)
                : "memory");
 }
+// Bulk prefetch of a contiguous global range into L2 (16-B aligned, size a multiple of 16 B)
+__device__ __forceinline__ void bulk_prefetch_l2(const void* src, uint32_t bytes) {
+  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
+}
 // 1-D bulk copy global -> shared (size multiple of 16 B, 16-B aligned), completes on an mbarrier
 __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, uint32_t bytes,
                                              uint64_t* bar) {

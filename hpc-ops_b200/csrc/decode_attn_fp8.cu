@@ -172,17 +172,44 @@ __global__ void __launch_bounds__(kThreads, 1)
       const int kc2 = p.k_head_first ? 0 : t.ihead_kv;
       const int vc1 = p.v_head_first ? t.ihead_kv : 0;
       const int vc2 = p.v_head_first ? 0 : t.ihead_kv;
+      // L2 prefetch duty: the Hkv CTAs that stream tile x of request b (one per kv head) do so in
+      // about the same step of the rotated walk; the one with ihead_kv == (b + x) % Hkv fetches
+      // that tile's two pages, K and V of all heads, into L2 pf_dist tiles before it loads tile x
+      // itself, so DRAM sees each page as one contiguous read. Only tiles of the current segment
+      // are prefetched: its first pf_dist tiles get none. pf_dist < 0: no prefetch.
+      const int pf_dist = p.pf_dist;
+      const int pf_phase = (__shfl_sync(0xffffffffu, t.ibatch + t.iseq_start / kTileN, 0) + pf_dist) %
+                           p.num_head_kv;
       for (int g0 = sg.tb; g0 < ntiles; g0 += 16) {
         int bi = g0 * 2 + lane;
         bi = bi < nblk ? bi : nblk - 1;  // a missing 2nd page of the last tile re-reads the 1st
         const int my_id = __ldg(ids + bi);
+        int pf_id = my_id;  // page ids pf_dist tiles ahead, same lane order
+        if (pf_dist > 0) {  // (distance 0: the ids of the tiles loaded now)
+          int pbi = (g0 + pf_dist) * 2 + lane;
+          pbi = pbi < nblk ? pbi : nblk - 1;
+          pf_id = __ldg(ids + pbi);
+        }
         const int gt = (ntiles - g0) < 16 ? (ntiles - g0) : 16;
         for (int tt = 0; tt < gt; tt++) {
           const int id0 = __shfl_sync(0xffffffffu, my_id, 2 * tt);
           const int id1 = __shfl_sync(0xffffffffu, my_id, 2 * tt + 1);
+          const int pf0 = __shfl_sync(0xffffffffu, pf_id, 2 * tt);
+          const int pf1 = __shfl_sync(0xffffffffu, pf_id, 2 * tt + 1);
+          const int pt = g0 + tt + pf_dist;  // tile of the task to prefetch
+          const bool pf = pf_dist >= 0 && pt < ntiles &&
+                          (pf_phase + g0 + tt) % p.num_head_kv == t.ihead_kv;
           const uint32_t st = n % kNumStages;
           mbar_wait(&stage_empty[st], ((n / kNumStages) & 1) ^ 1);
           if (elect_one()) {
+            if (pf) {
+              bulk_prefetch_l2(p.pf_k + pf0 * p.pf_k_blk, p.pf_bytes);
+              bulk_prefetch_l2(p.pf_v + pf0 * p.pf_v_blk, p.pf_bytes);
+              if (2 * pt + 1 < nblk) {
+                bulk_prefetch_l2(p.pf_k + pf1 * p.pf_k_blk, p.pf_bytes);
+                bulk_prefetch_l2(p.pf_v + pf1 * p.pf_v_blk, p.pf_bytes);
+              }
+            }
             uint8_t* dst = stages + st * kStageBytes;
             mbar_arrive_expect_tx(&k_full[st], kSlotBytes);
             tma_load_4d_hint(dst, &tmap_k, &k_full[st], 0, kc1, kc2, id0, pol_stream);
@@ -688,6 +715,18 @@ static int decode_fp8_impl(
                 (reinterpret_cast<uintptr_t>(vcache_ptr) % 256) == 0;
   if (const char* e = getenv("HPC_B200_DECODE_ROTATE")) rotate = rotate && atoi(e) != 0;
 
+  // Page-wide L2 prefetch (producer warp): when each cache is dense token-major, one page's rows of
+  // all heads are one contiguous range, [blk * block_stride, + 64 * token_stride) (the k-per-token
+  // scale rows follow it and are not prefetched). One bulk prefetch per page, so at most 8 kv heads
+  // (64 KB, the size run on B200). HPC_B200_KV_PREFETCH=0 disables it, HPC_B200_KV_PREFETCH_DIST
+  // sets the distance in tiles.
+  const int64_t dense_row = static_cast<int64_t>(num_head_k) * 128;
+  bool prefetch = rotate && num_head_k <= 8 && kcache_token_stride == dense_row &&
+                  vcache_token_stride == dense_row;
+  if (const char* e = getenv("HPC_B200_KV_PREFETCH")) prefetch = prefetch && atoi(e) != 0;
+  int pf_dist = 1;
+  if (const char* e = getenv("HPC_B200_KV_PREFETCH_DIST")) pf_dist = atoi(e);
+
   CUtensorMap tq, tk, tv;
   {
     uint64_t dims[3] = {128, static_cast<uint64_t>(num_head_q),
@@ -730,7 +769,9 @@ static int decode_fp8_impl(
     // which is consumed by another CTA much later (measured: +49 % DRAM reads, profiles/).
     // ... unless the walk is rotated: then the neighbouring head's row is wanted by another CTA at
     // the same time and the wider fetch is its prefetch (decode_common.cuh).
-    CUtensorMapL2promotion promo = (tok_stride == 128 || rotate)
+    // With the page-wide prefetch the loads find their lines in L2 and the wider promotion only
+    // adds reads (measured at C2: 172 vs 173 us, profiles/decode_prefetch_ab.json).
+    CUtensorMapL2promotion promo = (tok_stride == 128 || (rotate && !prefetch))
                                        ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B
                                        : CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
     if (const char* e = getenv("HPC_B200_KV_PROMO")) {  // tuning knob: 0 none, 1 64B, 2 128B, 3 256B
@@ -783,6 +824,12 @@ static int decode_fp8_impl(
   // 180 vs 199 us, profiles/r2_decode_rotate_ab2.json)
   p.kv_policy = rotate ? 1 : 0;
   if (const char* e = getenv("HPC_B200_KV_POLICY")) p.kv_policy = atoi(e);  // tuning knob
+  p.pf_dist = prefetch && pf_dist >= 0 ? pf_dist : -1;
+  p.pf_bytes = static_cast<uint32_t>(64 * dense_row);
+  p.pf_k = static_cast<const uint8_t*>(kcache_ptr);
+  p.pf_v = static_cast<const uint8_t*>(vcache_ptr);
+  p.pf_k_blk = kcache_block_stride;
+  p.pf_v_blk = vcache_block_stride;
 
   const int grid = splitk;  // == num_total_ctas of the task map
   int rc;

@@ -40,6 +40,13 @@ struct Params {
   long long ks_blk, ks_row, ks_head;
   int rotate;  // walk each bin from the tile whose position on the per-head line is 0 (mod P)
   int kv_policy;  // L2 policy of the K/V loads: 0 evict_first, 1 evict_normal, 2 evict_last
+  // fp8 kernel, dense token-major caches under the rotated walk: page-wide L2 prefetch pf_dist
+  // tiles ahead (< 0: off). Page blk of K (all heads) is [pf_k + blk * pf_k_blk, + pf_bytes).
+  int pf_dist;
+  uint32_t pf_bytes;
+  const uint8_t* pf_k;
+  const uint8_t* pf_v;
+  long long pf_k_blk, pf_v_blk;
 };
 
 struct Task {
